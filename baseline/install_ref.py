@@ -3,8 +3,7 @@
 
 ``pip install /root/reference`` cannot work here: the six pybind11 extensions need Eigen, an un-vendored submodule that is
 missing (SURVEY section 8c), and ``probreg/__init__.py`` imports open3d / transforms3d, which are absent.  The CPD path
-itself is pure Python + numpy/scipy, so the files it consists of (and bcpd.py, whose host-side M-step the
-BCPD parity test needs run on the SAME host as the package: its float32 matrix inverse is machine-dependent) are copied byte for byte (checksums recorded in
+itself is pure Python + numpy/scipy, so the files it consists of are copied byte for byte (checksums recorded in
 ``baseline/_ref/MANIFEST.json``); nothing under ``baseline/_ref`` is tracked by git, and nothing in the product imports it.
 Runs only where ``/root/reference`` exists (the build container); the GPU box uses the copy that travelled with gpurun.
 """
@@ -15,7 +14,7 @@ import shutil
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-FILES = ["cpd.py", "bcpd.py", "transformation.py", "math_utils.py", "log.py", "version.py"]
+FILES = ["cpd.py", "transformation.py", "math_utils.py", "log.py", "version.py"]
 
 
 def install(ref="/root/reference", force=False):

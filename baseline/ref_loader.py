@@ -42,14 +42,6 @@ def load():
     m = types.ModuleType("probreg._math")
     m.squared_kernel = orc.squared_kernel_f32
     m.rbf_kernel = orc.rbf_kernel_f32
-    m.inverse_multiquadric_kernel = orc.imq_kernel_f32
     sys.modules["probreg._math"] = m
     pkg._math = m
     return importlib.import_module("probreg.cpd"), importlib.import_module("probreg.transformation")
-
-
-def load_bcpd():
-    """-> probreg.bcpd of the reference, unmodified (its host-side M-step inverts a float32 kernel matrix of condition ~1e10:
-    results are only comparable between runs on the same host and numpy build, which is why the GPU parity test runs it live)."""
-    load()
-    return importlib.import_module("probreg.bcpd")

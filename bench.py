@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- CPD EM-iterations/sec at N = M = 100k 3-D points on N B200s (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points 100000]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points 100000] [--dump-outputs DIR]
   N > 1 is launched by torchrun (one rank per GPU); rank 0 prints ONE JSON line.
 
 A "step" is one EM iteration (probreg/cpd.py:111-113: transform -> E-step -> M-step) of rigid CPD
@@ -257,11 +257,12 @@ def port_sample(points, cols):
     src, tgt = workload(points)
     s2 = float(orc.sigma2_init_exact(src, tgt))
     cols = min(cols, points)
+    sub = tgt[:cols]
     chunk = 250
     orc.expectation_step(src, tgt[:chunk], s2, 0.0, n_global=points)          # untimed: see reference_sample
     t0 = time.perf_counter()
     ts = orc.apply_rigid(src, np.identity(3), np.zeros(3))
-    parts = [orc.expectation_step(ts, tgt[lo:lo + chunk], s2, 0.0, n_global=points) for lo in range(0, cols, chunk)]
+    parts = [orc.expectation_step(ts, sub[lo:lo + chunk], s2, 0.0, n_global=points) for lo in range(0, cols, chunk)]
     es = orc.Estep(np.concatenate([e.pt1 for e in parts]), sum(e.p1 for e in parts), sum(e.px for e in parts),
                    float(sum(e.p1.sum() for e in parts)))
     t_e = time.perf_counter() - t0
@@ -328,6 +329,8 @@ def run_ours(args):
 
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: probreg_b200 has no CPU path")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of a one-GPU run (each rank holds only its shard's sums)")
     torch.cuda.set_device(local_rank)
     comm = None
     if world > 1:
@@ -399,6 +402,11 @@ def run_ours(args):
     t_wall = t_wall1 - t_wall0
     launches = h.launch_count() - launches0
     clocks = sampler.stop(t_wall0, t_wall1, t_up) if sampler else None
+    if args.dump_outputs:
+        lin, t, scale, sigma2, q, n_p, _ = h.em_run(0, 0.0)        # maxiter 0: the state the last step left, no further step
+        pt1, p1, px, _ = h.last_estep()
+        dump_outputs(args.dump_outputs, {"lin": lin, "t": t, "scale": scale, "sigma2": sigma2, "q": q, "n_p": n_p,
+                                         "pt1": pt1, "p1": p1, "px": px})
     per_step = np.array([h.event_elapsed(2 * i, 2 * i + 1) for i in range(args.steps)])
     total_ms = float(per_step.sum())
     if world > 1:
@@ -644,6 +652,8 @@ def run_nonrigid(args, torch, _cabi, cpd, barrier, local_rank, world):
     t_wall1 = time.perf_counter()
     launches = h.launch_count() - launches0
     clocks = sampler.stop(t_wall0, t_wall1, t_up) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sigma2": sig, "w": h.nonrigid_w(), "moved": h.nonrigid_moved()})
     per_step = np.array([h.event_elapsed(2 * i, 2 * i + 1) for i in range(args.steps)])
     ms_per_step = float(per_step.sum()) / args.steps
     h.set_profiling(True)
@@ -725,6 +735,28 @@ def run_extras():
         return {"error": "%s: %s" % (type(e).__name__, str(e)[:300])}
 
 
+DUMP_BYTES = 63 * 10 ** 6       # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: write `arrays` as <path>/<name>.npy in float64, so that two builds run with the same arguments can be compared
+    output for output.  Past DUMP_BYTES in all, every array of more than 1 MiB keeps the same share of its rows, a sample drawn with
+    seed 0 from its row count alone: arrays with the same rows (p1 and px) keep the same rows, and so does a second build."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    big = [k for k, a in arrays.items() if a.nbytes > 1 << 20]
+    small_bytes = sum(a.nbytes for k, a in arrays.items() if k not in big)
+    big_bytes = sum(arrays[k].nbytes for k in big)
+    if small_bytes + big_bytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - small_bytes) / float(big_bytes)
+        for k in big:
+            n = arrays[k].shape[0]
+            rows = np.sort(np.random.default_rng(0).choice(n, max(1, int(n * keep)), replace=False))
+            arrays[k] = arrays[k][rows]
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def emit(obj):
     """The ONE JSON line goes to the real stdout; everything else this process (or NCCL, which
     prints its version banner to fd 1) writes during the run has been diverted to stderr."""
@@ -748,7 +780,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-also", action="store_true", help="skip the short runs of configurations 3 and 5 reported under config.also")
     ap.add_argument("--extras", action="store_true", help="add the side measurements of tools/bench_extras.py (key \"extras\")")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                                                          "(float64; one GPU, --impl ours)")
     args = ap.parse_args()
+    if not 1 <= args.steps <= 4096:
+        ap.error("--steps must be in 1 .. 4096 (each timed step takes two of the library's 8192 event slots)")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.kind = WORKLOADS[args.config][0]
     if args.points <= 0:
         args.points = WORKLOADS[args.config][1]

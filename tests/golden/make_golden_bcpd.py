@@ -60,7 +60,10 @@ def main():
     out["reg_source"], out["reg_target"] = s_small, t_small
     out["reg_rot"], out["reg_t"], out["reg_scale"], out["reg_v"] = tfm.rigid_trans.rot, tfm.rigid_trans.t, tfm.rigid_trans.scale, tfm.v
     np.savez_compressed(os.path.join(HERE, "bcpd.npz"), **out)
-    print("wrote bcpd.npz")
+    # the float32 inverse of the kernel matrix that registration used (condition ~1e10: LAPACK's result depends on the CPU and the
+    # thread count), so that the test can hand the same inverse to the package and compare the rest on any host
+    np.savez_compressed(os.path.join(HERE, "bcpd_gmat_inv.npz"), gmat_inv=reg.gmat_inv)
+    print("wrote bcpd.npz, bcpd_gmat_inv.npz")
 
 
 if __name__ == "__main__":

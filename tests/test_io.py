@@ -1,13 +1,14 @@
-"""probreg_b200.io: readers and the voxel down-sampler (CPU; the optional part uses the reference's data when present)."""
+"""probreg_b200.io: readers and the voxel down-sampler (CPU; also on the reference's example data, kept under tests/golden/ref_data)."""
 import os
 import struct
 
 import numpy as np
 import pytest
 
+from conftest import GOLDEN
 from probreg_b200 import io as pio
 
-REF = "/root/reference"
+REF_DATA = os.path.join(GOLDEN, "ref_data")
 
 
 def test_pcd_and_txt_roundtrip(tmp_path):
@@ -48,19 +49,20 @@ def test_voxel_down_sample():
         pio.voxel_down_sample(cloud, 0.0)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
 def test_reference_fixtures_load():
-    bunny = pio.read_points(os.path.join(REF, "examples", "bunny.pcd"))
+    bunny = pio.read_points(os.path.join(REF_DATA, "bunny.pcd"))
     assert bunny.shape == (397, 3)                                            # examples/bunny.pcd:9
     assert abs(pio.voxel_down_sample(bunny, 0.005).shape[0] - 381) <= 12      # SURVEY: ~381 points at voxel 0.005
-    horse = pio.read_points(os.path.join(REF, "data", "horse.ply"))
-    assert horse.shape == (48485, 3)                                          # binary_big_endian, 48 485 vertices
+    # data/horse.ply (binary_big_endian, 48 485 vertices) shrunk to one vertex per occupied voxel of the 0.01 grid, which keeps
+    # the full file's voxel count (tests/golden/make_ref_data.py)
+    horse = pio.read_points(os.path.join(REF_DATA, "horse.ply"))
+    assert horse.shape == (490, 3)
     assert abs(pio.voxel_down_sample(horse, 0.01).shape[0] - 480) <= 40       # tests/test_cpd.py recipe: ~480 points
-    assert pio.read_points(os.path.join(REF, "examples", "cloud_0.pcd")).shape == (6535, 3)
-    assert pio.read_points(os.path.join(REF, "examples", "fish_source.txt")).shape == (91, 2)
+    assert pio.read_points(os.path.join(REF_DATA, "cloud_0.pcd")).shape == (500, 3)      # the first 500 of 6 535 points
+    assert pio.read_points(os.path.join(REF_DATA, "fish_source.txt")).shape == (91, 2)
 
 
-def test_example_utils_follow_the_reference_recipes():
+def test_example_utils_follow_the_reference_recipes(monkeypatch):
     """examples/utils.py: numpy counterparts of the reference's examples/utils.py (rigid recipe: voxel filter, shuffle, noise,
     outliers, 30 degrees about z; non-rigid: the two text clouds, voxel-filtered)."""
     import os
@@ -74,9 +76,9 @@ def test_example_utils_follow_the_reference_recipes():
     r = ex.euler2mat(0.1, -0.2, 0.3)
     np.testing.assert_allclose(r.dot(r.T), np.identity(3), atol=1e-15)
     np.testing.assert_allclose(ex.euler2mat(0.0, 0.0, np.deg2rad(30.0))[:2, :2], [[np.cos(np.pi / 6), -0.5], [0.5, np.cos(np.pi / 6)]], atol=1e-15)
+    monkeypatch.setenv("PROBREG_EXAMPLES", REF_DATA)
     bunny = ex.reference_file("bunny.pcd")
-    if bunny is None:
-        return                                                          # the reference's data files are not around (GPU box)
+    assert bunny is not None
     src, tgt = ex.prepare_source_and_target_rigid_3d(bunny, rng=np.random.default_rng(0))
     assert src.shape[1] == 3 and tgt.shape == (src.shape[0] + 500, 3)
     # undo the known transform: the inliers are the (shuffled, slightly noised) source
