@@ -4,7 +4,6 @@
 #include "cpd_b200.h"
 #include "kernels.cuh"
 #include "lowrank.cuh"
-#include "gram_umma.cuh"
 #include "gram_i8.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -224,8 +223,6 @@ struct cpd_ctx {
            *d_lr_R = nullptr, *d_lr_sys = nullptr, *d_lr_rhs = nullptr, *d_lr_c = nullptr, *d_lr_out = nullptr, *d_lr_panel = nullptr, *d_lr_Lt = nullptr;
     bool lr_spd = true;                   // symmetric positive definite K x K system on Qt = Q L (lr_spd_form); CPD_B200_LR_CORE=lu: LU of (c I + Bc S)
     size_t lr_part_cap = 0;               // doubles in d_lr_part (slice partials of lr_inner)
-    float *d_gu_planes = nullptr, *d_gu_part = nullptr;      // tcgen05 G X product: TF32 hi / lo planes of X, chunk partials
-    size_t gu_planes_cap = 0, gu_part_cap = 0;
     unsigned char* d_gi_planes = nullptr;                      // exact int8-digit product: digit planes of X, FP64 chunk partials, column maxima
     double *d_gi_part = nullptr, *d_gi_colmax = nullptr;
     size_t gi_planes_cap = 0, gi_part_cap = 0, gi_colmax_cap = 0, gi_pairs_cap = 0;
@@ -670,7 +667,7 @@ extern "C" void cpd_destroy(cpd_ctx* h) {
     void* nrp[] = {h->d_G, h->d_W, h->d_A, h->d_B, h->d_ts2, h->d_nrpart, h->d_ipiv, h->d_info, h->d_work};
     for (void* p : nrp) if (p) cudaFree(p);
     void* lrp[] = {h->d_lr_pts, h->d_lr_Q, h->d_lr_X, h->d_lr_coef, h->d_lr_part, h->d_lr_Bc, h->d_lr_S, h->d_lr_R, h->d_lr_sys, h->d_lr_rhs,
-                   h->d_lr_c, h->d_lr_out, h->d_lr_panel, h->d_lr_Lt, h->d_gu_planes, h->d_gu_part, h->d_gi_planes, h->d_gi_part, h->d_gi_colmax, h->d_gi_pairs, h->d_wgt, h->d_p1t, h->d_pxt, h->d_la, h->d_log2c};
+                   h->d_lr_c, h->d_lr_out, h->d_lr_panel, h->d_lr_Lt, h->d_gi_planes, h->d_gi_part, h->d_gi_colmax, h->d_gi_pairs, h->d_wgt, h->d_p1t, h->d_pxt, h->d_la, h->d_log2c};
     for (void* p : lrp) if (p) cudaFree(p);
     if (h->h_work) free(h->h_work);
     if (h->sol_params && g_sol.DestroyParams) g_sol.DestroyParams(h->sol_params);

@@ -436,12 +436,11 @@ np.save(sys.argv[1], q.dot(b).dot(q.T))
 
 @pytest.mark.gpu
 @pytest.mark.timeout(900)
-def test_every_selectable_gram_product_gives_the_same_factorisation(tmp_path):
-    """CPD_B200_LR_GRAM selects the kernel behind the G X products of the range finder: the exact integer-digit tensor-core kernels
-    (A operand in tensor memory -- the default -- or in shared memory), the TF32 x 3 tensor-core kernel, the CUDA-core kernel.  The
-    variable is read once per process, hence subprocesses.  The two integer kernels and the CUDA-core kernel agree with the float32
-    G of the reference to 1e-6 (relative, spectral norm); the TF32 kernel to the 3e-5 its truncating FP32 accumulation in TMEM
-    allows (DESIGN 4c) -- which is why it is not the default.  A rank of 130 takes two column passes, 1300 points 11 row tiles."""
+def test_i8_and_simt_gram_products_agree_and_other_modes_are_refused(tmp_path):
+    """CPD_B200_LR_GRAM selects the kernel behind the G X products of the range finder: the exact integer-digit tensor-core kernel
+    (i8, the default) or the CUDA-core kernel (simt).  The variable is read once per process, hence subprocesses.  Both agree with
+    the float32 G of the reference to 1e-6 (relative, spectral norm).  Any other value is refused with an error that names the
+    accepted ones, never silently replaced by the default.  A rank of 130 takes two column passes, 1300 points 11 row tiles."""
     import subprocess
     import sys
 
@@ -452,11 +451,15 @@ def test_every_selectable_gram_product_gives_the_same_factorisation(tmp_path):
     g = orc.rbf_kernel_f32(src, src, beta).astype(np.float64)
     code = _PRODUCT_SCRIPT % (ROOT, m, beta, rank)
     errs = {}
-    for mode in ("i8", "i8ss", "simt", "tf32"):
+    for mode in ("i8", "simt"):
         out = str(tmp_path / ("g_%s.npy" % mode))
         r = subprocess.run([sys.executable, "-c", code, out], capture_output=True, text=True, timeout=600,
                            env=dict(os.environ, CPD_B200_LR_GRAM=mode))
         assert r.returncode == 0, (mode, r.stderr[-2000:])
         errs[mode] = np.linalg.norm(np.load(out) - g, 2) / np.linalg.norm(g, 2)
-    assert errs["i8"] < 1e-6 and errs["i8ss"] < 1e-6 and errs["simt"] < 1e-6, errs
-    assert errs["tf32"] < 3e-5, errs
+    assert errs["i8"] < 1e-6 and errs["simt"] < 1e-6, errs
+    out = str(tmp_path / "g_tf32.npy")
+    r = subprocess.run([sys.executable, "-c", code, out], capture_output=True, text=True, timeout=600,
+                       env=dict(os.environ, CPD_B200_LR_GRAM="tf32"))
+    assert r.returncode != 0 and not os.path.exists(out), r.stdout[-2000:]
+    assert "CPD_B200_LR_GRAM=tf32: the accepted values are i8 (the default) and simt (code -1)" in r.stderr, r.stderr[-2000:]
